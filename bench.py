@@ -3,8 +3,13 @@
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
                     [--config fbocc200|unit|frames16|bwd_only|large]
+                    [--dump-outputs DIR]
 
-A *step* is one pass of the hot path over one batch of synthetic input.  The
+A *step* is one pass of the hot path over one batch of synthetic input; every
+timed pass runs K of them.  The inputs are seeded, so the same arguments give
+the same inputs on every run, and `--dump-outputs DIR` writes what the last
+timed step returned (rank 0) as DIR/<name>.npy: two builds of the project
+can then be compared output for output.  The
 default workload is BASELINE.json configs[1] (FB-OCC R50 single frame: 6
 cameras 256x704, feature map 16x44, D = 80 depth bins, C = 80, 200x200x16 voxel
 grid, 200x200 BEV queries, 8 heads, 1 level, 8 points, 4 Z anchors), one frame
@@ -44,6 +49,8 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+# the benchmark leaves the tree as it found it (it may be read-only)
+sys.dont_write_bytecode = True
 
 import numpy as np  # noqa: E402
 import torch  # noqa: E402
@@ -241,6 +248,8 @@ class Workload:
 
     @torch.no_grad()
     def step(self):
+        """-> the step's results, also kept as ``last_out`` (under a CUDA
+        graph: the graph's output tensors, which every replay rewrites)."""
         outs = []
         if self.vt is not None:
             outs.append(self.vt(self.cam, self.feat, self.depth))  # (B,C,Y,X,Z)
@@ -249,7 +258,12 @@ class Workload:
                                 lss_bev=self.lss, cam_params=self.cam,
                                 pred_img_depth=self.depth,
                                 out=self.out_buffer))
-        return tuple(outs)
+        self.last_out = tuple(outs)
+        return self.last_out
+
+    def out_names(self):
+        return (["bev_volume"] if self.vt is not None else []) + \
+            (["bev_refined"] if self.bp is not None else [])
 
     def capture(self, after=None):
         """Capture one step (the plugin forwards, plus `after()` when given --
@@ -645,6 +659,29 @@ def timed_steps(fn, steps, flush, barrier):
     return sum(s.elapsed_time(e) for s, e in events) / steps
 
 
+DUMP_BYTES = 60 << 20
+
+
+def dump_outputs(outs, names, out_dir):
+    """Write each result as out_dir/<name>.npy (float32), DUMP_BYTES in all.
+    Smaller results are written whole and first; a result beyond what is left
+    of the budget is written as the elements at flat indices drawn by a
+    generator seeded with 0 (the same on every run), as <name>_sample.npy."""
+    os.makedirs(out_dir, exist_ok=True)
+    left = DUMP_BYTES // 4
+    order = sorted(range(len(outs)), key=lambda i: outs[i].numel())
+    for k, i in enumerate(order):
+        t, name = outs[i].detach(), names[i]
+        cap = left // (len(outs) - k)
+        if t.numel() > cap:
+            g = torch.Generator().manual_seed(0)
+            idx = torch.randint(t.numel(), (cap,), generator=g)
+            t, name = t.reshape(-1)[idx.to(t.device)], name + "_sample"
+        np.save(os.path.join(out_dir, name + ".npy"),
+                t.float().cpu().numpy())
+        left -= t.numel()
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -665,7 +702,17 @@ def main():
     ap.add_argument("--eager-only", action="store_true",
                     help="profiling aid: stop after the eager pass (what ncu "
                          "captures) and print only its numbers")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the results of the "
+                         "last one as DIR/<name>.npy (rank 0; at most 64 MB "
+                         "in all, a larger result as a fixed seeded sample)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl == "reference" or args.kernels_only
+                              or args.eager_only):
+        ap.error("--dump-outputs writes the results of the headline pass: "
+                 "not with --impl reference, --kernels-only or --eager-only")
     if args.impl == "reference":
         # CPU arm: rank 0 alone works, the other ranks of a torchrun launch
         # exit at once; no process group is needed
@@ -706,7 +753,7 @@ def main():
     # spin kernel keeps the GPU busy while the step's launches queue up, so the
     # intervals are device execution back to back (as in the graph replay), not
     # host launch gaps ---------------------------------------------------------
-    ksteps = max(3, min(args.steps, 10))
+    ksteps = args.steps
     with _lib.KernelTimer() as kt:
         for _ in range(ksteps):
             flush.zero_()
@@ -750,11 +797,13 @@ def main():
     step_ms = timed_steps(run_step, args.steps, flush, barrier)
     wall = time.perf_counter() - wall0
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(w.last_out, w.out_names(), args.dump_outputs)
 
     # ---- end to end: pinned host inputs -> plugin calls -> host results ----
     outs = w.step()
     host_out = [torch.empty(t.shape, dtype=t.dtype).pin_memory() for t in outs]
-    e2e_steps = max(3, min(args.steps, 10))
+    e2e_steps = args.steps
 
     def e2e_step():
         if use_graph:
@@ -813,7 +862,7 @@ def main():
     if (args.config == "fbocc200" and not args.no_frames16 and 16 % world == 0):
         try:
             extra["frames16"] = frames16_block(world, rank, dev, flush, barrier,
-                                               max(3, min(args.steps, 10)))
+                                               args.steps)
         except Exception as ex:
             extra["frames16"] = {"unavailable": str(ex)[:160]}
 

@@ -1,9 +1,11 @@
 """ctypes binding of ``oracle/_ref/libbev_pool_ref.so`` -- the reference's OWN
 ``bev_pool_cuda.cu`` compiled for sm_100a by ``oracle/Makefile`` (GPU box only).
 
-TEST INFRASTRUCTURE ONLY -- see ``oracle/__init__.py``.  Used by the ``-m gpu``
-parity tests (CUDA path vs the unmodified reference kernels on identical
-inputs) and by ``bench.py`` for the "reference CUDA kernel on this B200" line.
+TEST INFRASTRUCTURE ONLY -- see ``oracle/__init__.py``.  Used by
+``tests/golden/gen_golden_ref_kernel.py`` to record the outputs the ``-m gpu``
+parity tests compare the CUDA path with (the unmodified reference kernels on
+identical inputs) and by ``bench.py`` for the "reference CUDA kernel on this
+B200" line.
 The reference launches on the legacy default stream
 (bev_pool_cuda.cu:124, 133); callers synchronise around it.
 """

@@ -3,9 +3,10 @@
 * ``-m "not gpu"``: oracle vs golden vectors, host logic, C-ABI load/export
   checks, world_size-2 gloo tests -- runs anywhere in a few minutes.
 * ``-m gpu``: the parity tests proper; they call the CUDA path through the
-  C ABI (ctypes) and compare with the oracle / golden fixtures.  They never
-  read /root/reference.
+  C ABI (ctypes) and compare with the oracle / golden fixtures.  They read
+  nothing outside the repository.
 """
+import glob
 import os
 import sys
 
@@ -42,9 +43,15 @@ def oracle_cpu():
 
 
 def load_golden(name):
-    path = os.path.join(GOLDEN, name + ".npz")
-    with np.load(path) as z:
-        return {k: z[k] for k in z.files}
+    """Arrays of fixture `name`: ``name.npz`` plus, for a fixture stored in
+    parts to keep every file below 1 MB, ``name.part1.npz``, ... ."""
+    paths = [os.path.join(GOLDEN, name + ".npz")] + sorted(
+        glob.glob(os.path.join(GOLDEN, glob.escape(name) + ".part*.npz")))
+    out = {}
+    for path in paths:
+        with np.load(path) as z:
+            out.update({k: z[k] for k in z.files})
+    return out
 
 
 def canon_index(ranks_bev, ranks_depth, ranks_feat):

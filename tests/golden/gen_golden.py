@@ -43,11 +43,26 @@ def _np(t):
     return None if t is None else t.detach().cpu().numpy()
 
 
+PART_BYTES = 900_000
+
+
 def save(name, **arrays):
-    path = os.path.join(HERE, name + ".npz")
+    """Write ``name.npz``; arrays beyond PART_BYTES go on into
+    ``name.part1.npz``, ... so every stored file stays below 1 MB
+    (conftest.load_golden merges the parts)."""
     arrays = {k: v for k, v in arrays.items() if v is not None}
-    np.savez_compressed(path, **arrays)
-    print(f"wrote {path}  ({os.path.getsize(path) / 1024:.1f} KiB)")
+    parts, size = [{}], 0
+    for k, v in arrays.items():
+        if parts[-1] and size + v.nbytes > PART_BYTES:
+            parts.append({})
+            size = 0
+        parts[-1][k] = v
+        size += v.nbytes
+    for i, part in enumerate(parts):
+        path = os.path.join(HERE, name + (f".part{i}" if i else "") + ".npz")
+        np.savez_compressed(path, **part)
+        assert os.path.getsize(path) < 1_000_000, path
+        print(f"wrote {path}  ({os.path.getsize(path) / 1024:.1f} KiB)")
 
 
 def gen_forward(ref):
