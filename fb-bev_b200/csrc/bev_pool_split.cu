@@ -36,6 +36,7 @@
 #include <cstdlib>
 
 #include "bev_pool_split.h"
+#include "bulk.cuh"
 
 namespace fbbev {
 
@@ -46,16 +47,6 @@ namespace fbbev {
 #define FBBEV_SUM_MINB 6
 #endif
 constexpr int kSumThreads = FBBEV_SUM_THREADS;  // interval-sum CTAs
-
-__device__ __forceinline__ void cp_async16(void* sdst, const void* gsrc) {
-  const uint32_t s = static_cast<uint32_t>(__cvta_generic_to_shared(sdst));
-  asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(s), "l"(gsrc)
-               : "memory");
-}
-__device__ __forceinline__ void cp_async_commit_wait_all() {
-  asm volatile("cp.async.commit_group;" ::: "memory");
-  asm volatile("cp.async.wait_group 0;" ::: "memory");
-}
 
 // ------------------------------- plan --------------------------------------
 // tile_first[t] = first interval of tile t (tile_first[n_tiles] = n);
@@ -360,7 +351,8 @@ __global__ void __launch_bounds__(2 * T, 1280 / (2 * T)) dense_write_kernel(
     const float4* src = reinterpret_cast<const float4*>(V) + (int64_t)i0 * c4;
     for (int r = warp; r < nrows; r += kWrWarps)
       for (int v = lane; v < c4; v += kWarp)
-        cp_async16(rows + (size_t)r * pitch + 4 * v, src + (size_t)r * c4 + v);
+        cp_async16(smem_u32(rows + (size_t)r * pitch + 4 * v),
+                   src + (size_t)r * c4 + v);
   }
   for (int q = tid; q < T; q += kWrThreads) slot[q] = T;
   for (int q = tid; q < pitch; q += kWrThreads) rows[(size_t)T * pitch + q] = 0.f;
@@ -378,7 +370,8 @@ __global__ void __launch_bounds__(2 * T, 1280 / (2 * T)) dense_write_kernel(
     carry_n[r] = nx;
     any_carry |= nx > 0;
   }
-  cp_async_commit_wait_all();
+  cp_async_commit();
+  cp_async_wait0();
   if (__syncthreads_or(any_carry)) {
     // add the carry rows of intervals that span several K1 slices, in slice
     // order (deterministic); one warp per row, 8 loads in flight per lane

@@ -1,19 +1,24 @@
-// bulk.cuh -- mbarrier + 1-D bulk-copy (TMA, cp.async.bulk) wrappers shared by
-// the kernels that stage contiguous global slabs in shared memory.
+// bulk.cuh -- PTX wrappers for mbarriers, 1-D bulk copies (TMA,
+// cp.async.bulk) and 16-byte cp.async, shared by every kernel that stages
+// global data in shared memory.
 #pragma once
 #include <stdint.h>
 
 namespace fbbev {
-namespace bulk {
 
-__device__ __forceinline__ uint32_t smem_addr(const void* p) {
+__device__ __forceinline__ uint32_t smem_u32(const void* p) {
   return static_cast<uint32_t>(__cvta_generic_to_shared(p));
 }
+
+// ---------------------------------- mbarrier ---------------------------------
 __device__ __forceinline__ void mbar_init(uint32_t bar, uint32_t count) {
   asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count));
 }
 __device__ __forceinline__ void fence_mbar_init() {
   asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+}
+__device__ __forceinline__ void mbar_arrive(uint32_t bar) {
+  asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory");
 }
 __device__ __forceinline__ void mbar_arrive_expect_tx(uint32_t bar, uint32_t tx) {
   asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar),
@@ -45,16 +50,57 @@ __device__ __forceinline__ bool mbar_test(uint32_t bar, uint32_t parity) {
       : "memory");
   return done != 0;
 }
+
+// ------------------------------ 1-D bulk copies -------------------------------
+// orders this thread's generic-proxy shared-memory writes before its later
+// async-proxy accesses (bulk copies, tcgen05.mma operand reads)
+__device__ __forceinline__ void fence_proxy_async() {
+  asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+}
 // global -> shared, `bytes` a multiple of 16, both addresses 16-byte aligned;
 // completion is signalled on `bar` as transaction bytes
-__device__ __forceinline__ void g2s(uint32_t dst, const void* src, uint32_t bytes,
-                                    uint32_t bar) {
+__device__ __forceinline__ void bulk_g2s(uint32_t dst, const void* src,
+                                         uint32_t bytes, uint32_t bar) {
   asm volatile(
       "cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes "
       "[%0], [%1], %2, [%3];" ::"r"(dst),
       "l"(src), "r"(bytes), "r"(bar)
       : "memory");
 }
+// shared -> global, same size / alignment rules; tracked by the issuing
+// thread's bulk async-group
+__device__ __forceinline__ void bulk_s2g(void* dst, uint32_t src, uint32_t bytes) {
+  asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;" ::"l"(dst),
+               "r"(src), "r"(bytes)
+               : "memory");
+}
+__device__ __forceinline__ void bulk_commit() {
+  asm volatile("cp.async.bulk.commit_group;" ::: "memory");
+}
+__device__ __forceinline__ void bulk_wait_read0() {  // smem sources reusable
+  asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");
+}
+__device__ __forceinline__ void bulk_wait0() {       // stores complete
+  asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");
+}
 
-}  // namespace bulk
+// ------------------------------ 16-byte cp.async ------------------------------
+__device__ __forceinline__ void cp_async16(uint32_t dst, const void* src) {
+  asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(dst), "l"(src)
+               : "memory");
+}
+// copies the first `src_bytes` (0 or 16) of `src` and zero-fills the rest
+__device__ __forceinline__ void cp_async16_zfill(uint32_t dst, const void* src,
+                                                 uint32_t src_bytes) {
+  asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;" ::"r"(dst),
+               "l"(src), "r"(src_bytes)
+               : "memory");
+}
+__device__ __forceinline__ void cp_async_commit() {
+  asm volatile("cp.async.commit_group;" ::: "memory");
+}
+__device__ __forceinline__ void cp_async_wait0() {
+  asm volatile("cp.async.wait_group 0;" ::: "memory");
+}
+
 }  // namespace fbbev

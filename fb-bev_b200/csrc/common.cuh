@@ -28,6 +28,19 @@ void count_launch(int n = 1);
 
 static inline int64_t ceil_div64(int64_t a, int64_t b) { return (a + b - 1) / b; }
 
+// SM count of the current device, queried once (148, a B200's, if the query
+// fails).
+static inline int sm_count() {
+  static int n_sm = 0;
+  if (n_sm == 0) {
+    int dev = 0;
+    cudaGetDevice(&dev);
+    cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, dev);
+    if (n_sm <= 0) n_sm = 148;
+  }
+  return n_sm;
+}
+
 // Streaming (evict-first) 128-bit / 32-bit stores for write-once outputs.
 __device__ __forceinline__ void st_stream(float4* p, const float4& v) {
   __stcs(p, v);

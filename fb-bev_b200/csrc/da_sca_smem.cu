@@ -108,7 +108,7 @@ __device__ __forceinline__ float2 ld2(const float* p) {
     float2 v;
     asm("ld.shared.v2.f32 {%0, %1}, [%2];"
         : "=f"(v.x), "=f"(v.y)
-        : "r"(bulk::smem_addr(p)));
+        : "r"(smem_u32(p)));
     return v;
   }
   return __ldg(reinterpret_cast<const float2*>(p));
@@ -221,7 +221,7 @@ __device__ __forceinline__ void sca_pass(const ScaSmemParams& P, const ScaCtx& C
   for (int z = 0; z < kZ; ++z) dw[z] = __shfl_sync(kFull, dwz, (lane & ~7) | z);
   // the staged map is used as soon as its bulk copies have landed; until then
   // (the first ~10 us of the CTA) the same gathers go to the global original
-  if (!tile_ready) tile_ready = bulk::mbar_test(bulk::smem_addr(C.bar), 0);
+  if (!tile_ready) tile_ready = mbar_test(smem_u32(C.bar), 0);
   if (active) {
 #pragma unroll
     for (int p = 0; p < kPts; ++p) {          // point index = pp * Z + z (:563-570)
@@ -269,8 +269,8 @@ __global__ void __launch_bounds__(kScaThreads, 1) da_sca_smem_kernel(
   const long long spare = (long long)gridDim.x - P.n_pairs;
   if (threadIdx.x == 0) {
     s_total = 0; s_next = 0; s_left_n = 0; s_pair = -1;
-    bulk::mbar_init(bulk::smem_addr(bar), 1);
-    bulk::fence_mbar_init();
+    mbar_init(smem_u32(bar), 1);
+    fence_mbar_init();
   }
   __syncthreads();
   {  // total of all partial counts
@@ -316,11 +316,11 @@ __global__ void __launch_bounds__(kScaThreads, 1) da_sca_smem_kernel(
   const int bn = pair;                        // value / depth are (b, n) major
 
   if (threadIdx.x == 0) {
-    const uint32_t barrier = bulk::smem_addr(bar);
-    bulk::mbar_arrive_expect_tx(barrier, (uint32_t)tile_bytes);
+    const uint32_t barrier = smem_u32(bar);
+    mbar_arrive_expect_tx(barrier, (uint32_t)tile_bytes);
     const char* src = reinterpret_cast<const char*>(
         P.value + (int64_t)bn * P.n_value * kE);
-    const uint32_t dst = bulk::smem_addr(tile);
+    const uint32_t dst = smem_u32(tile);
     // the K CTAs of a camera all pull the same 225 KB: start each one at a
     // different chunk so that they do not queue on the same L2 lines
     constexpr int kChunk = 8192;
@@ -329,7 +329,7 @@ __global__ void __launch_bounds__(kScaThreads, 1) da_sca_smem_kernel(
     for (int c = 0; c < n_chunks; ++c) {
       const int off = ((start + c) % n_chunks) * kChunk;
       const int nb = min(kChunk, tile_bytes - off);
-      bulk::g2s(dst + off, src + off, (uint32_t)nb, barrier);
+      bulk_g2s(dst + off, src + off, (uint32_t)nb, barrier);
     }
   }
 
@@ -392,7 +392,7 @@ __global__ void __launch_bounds__(kScaThreads, 1) da_sca_smem_kernel(
   }
   // the bulk copies must have landed before the CTA (and its shared memory)
   // goes away, also when this warp never touched the tile
-  if (!tile_ready) bulk::mbar_wait(bulk::smem_addr(bar), 0);
+  if (!tile_ready) mbar_wait(smem_u32(bar), 0);
 }
 
 size_t da_sca_smem_workspace_bytes(int bs, int n_cams) {
@@ -424,9 +424,7 @@ int da_sca_smem_launch(const float* value, const float* depth_prob,
   P.bs = bs; P.n_cams = n_cams; P.nq = nq; P.n_value = n_value;
   P.DC = DC; P.n_pairs = bs * n_cams;
 
-  int dev = 0, n_sm = 148;
-  cudaGetDevice(&dev);
-  cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, dev);
+  const int n_sm = sm_count();
   const int64_t n_out4 = (int64_t)bs * nq * kE / 4;
   const int zero_blocks = (int)std::min<int64_t>(ceil_div64(n_out4, 256 * 4),
                                                  (int64_t)n_sm * 16);

@@ -43,47 +43,20 @@
 // (4 x 25.6 KB) | barriers, biases, LayerNorm parameters.
 // TMEM columns: H [0, hidden) | Y [hidden, hidden + pad16(E)) | lo ring 2 x 40.
 //
-// Shapes: E <= 80, E % 4 == 0; hidden % 80 == 0, hidden + pad16(E) + 80 <= 512.
-#include "common.cuh"
+// Shapes: E <= 80, E % 4 == 0; hidden % 80 == 0, hidden <= 320 (the b1 staged in
+// shared memory), hidden + pad16(E) + 80 <= 512.
 #include "tc5.cuh"
 
 namespace fbbev {
 namespace ffn {
 
-constexpr int kKB = 40;                 // floats of K per block
-constexpr int kChunks = kKB / 4;        // 16-byte chunks of a row per K-block
-constexpr int kTileM = 128;
-constexpr int kAPart = kTileM * kKB * 4;            // bytes of A_hi (== A_lo)
-constexpr int kABlock = 2 * kAPart;                 // one K-block, hi + lo
-constexpr int kAChunkStride = (kTileM / 8) * 128;   // bytes between K chunks
+constexpr int kABlock = 2 * kAPart;     // one K-block of X, hi + lo
 constexpr int kThreads = 448;
 constexpr int kHC = 80;                 // hidden columns per GEMM1 chunk
 constexpr int kMaxE = 80;
 constexpr int kMaxHidden = 320;
-constexpr int kTmemCols = 512;
-constexpr int kSmemLimit = 232448 - 1024;
 constexpr int kCtrlBytes = 512 + (kMaxHidden + 3 * kMaxE) * 4;
 constexpr int kSlabBytes = kTileM * (kMaxE + 4) * 4;
-
-#ifdef FFN_TRACE
-// timeline of CTA 0: every tracing thread (one per role) appends (tag, clock)
-// to its own region of a global buffer (plain stores, private counter)
-constexpr int kTraceCap = 200;
-__device__ long long g_ffn_trace[5 * 2 * kTraceCap];
-__device__ int g_ffn_trace_cnt[5];
-#define FTRACE_DECL int trn_ = 0;
-#define FTRACE_L(lane_, tag)                                                 \
-  do {                                                                       \
-    if (blockIdx.x == 0 && trn_ < kTraceCap) {                               \
-      g_ffn_trace[(lane_) * 2 * kTraceCap + 2 * trn_] = (tag);               \
-      g_ffn_trace[(lane_) * 2 * kTraceCap + 2 * trn_ + 1] = clock64();       \
-      g_ffn_trace_cnt[lane_] = ++trn_;                                       \
-    }                                                                        \
-  } while (0)
-#else
-#define FTRACE_DECL
-#define FTRACE_L(lane_, tag) do {} while (0)
-#endif
 
 struct Params {
   const float* x;         // [M][E]
@@ -102,7 +75,7 @@ struct Params {
 
 __global__ void __launch_bounds__(kThreads, 1) ffn_tf32_kernel(const Params p) {
   extern __shared__ __align__(1024) unsigned char smem[];
-  FTRACE_DECL
+  TRACE_DECL
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int npad = p.npad, S = p.wstages;
   const uint32_t w1_stage = 2u * kHC * kKB * 4;           // W1 chunk x K-block
@@ -145,13 +118,7 @@ __global__ void __launch_bounds__(kThreads, 1) ffn_tf32_kernel(const Params p) {
       fence_mbar_init();
     }
     __syncwarp();
-    asm volatile(
-        "tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(
-            smem_u32(tmem_slot)),
-        "r"(kTmemCols)
-        : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::
-                     : "memory");
+    tmem_alloc(smem_u32(tmem_slot));
   }
   for (int j = threadIdx.x; j < kMaxHidden; j += kThreads)
     s_b1[j] = (p.b1 && j < p.hidden) ? p.b1[j] : 0.f;
@@ -164,7 +131,7 @@ __global__ void __launch_bounds__(kThreads, 1) ffn_tf32_kernel(const Params p) {
   __syncthreads();
   tc_fence_after();
   const uint32_t tmem_base = *tmem_slot;
-  if (threadIdx.x == 0) FTRACE_L(4, 1);
+  if (threadIdx.x == 0) TRACE(4, 1);
   const int row_begin = blockIdx.x * p.rows_per_cta;
   const int row_end = min(p.M, row_begin + p.rows_per_cta);
   const int n_my = row_end > row_begin ? (row_end - row_begin + kTileM - 1) / kTileM : 0;
@@ -175,55 +142,23 @@ __global__ void __launch_bounds__(kThreads, 1) ffn_tf32_kernel(const Params p) {
     // the whole K range of a 128-row tile per round, through registers (hi / lo
     // split)
     const int lw = warp - 4;
-    const int r_lo = lane & 15, c_lo = lane >> 4;
     auto load_x = [&](int ti) {
       float4 v[2][10];
 #pragma unroll
-      for (int u = 0; u < 2; ++u) {
-        const int g0 = row_begin + ti * kTileM + lw * 32 + r_lo;
-        const int col0 = u * kKB + 4 * c_lo;
-        const float* b0 = p.x + (size_t)g0 * p.ldx + col0;
-        const float* b1 = b0 + (size_t)16 * p.ldx;
-        const bool ok0 = u < p.n_kb1 && g0 < row_end;
-        const bool ok1 = u < p.n_kb1 && g0 + 16 < row_end;
-#pragma unroll
-        for (int i = 0; i < 10; ++i) {
-          const int cp = i % 5;
-          const bool ok = (i < 5 ? ok0 : ok1) && col0 + 8 * cp < p.E;
-          v[u][i] = ok ? __ldg(reinterpret_cast<const float4*>(
-                             (i < 5 ? b0 : b1) + 8 * cp))
-                       : make_float4(0.f, 0.f, 0.f, 0.f);
-        }
-      }
-      if (threadIdx.x == 128) FTRACE_L(0, 100 + ti);
+      for (int u = 0; u < 2; ++u)
+        gather_kblock(v[u], p.x, p.ldx, nullptr, 0, p.E, row_begin + ti * kTileM,
+                      row_end, u, u < p.n_kb1, lw, lane);
+      if (threadIdx.x == 128) TRACE(0, 100 + ti);
       mbar_wait(bar_xempty, (ti & 1) ^ 1);   // GEMM1 of the previous tile done
-      if (threadIdx.x == 128) FTRACE_L(0, 110 + ti);
+      if (threadIdx.x == 128) TRACE(0, 110 + ti);
 #pragma unroll
       for (int u = 0; u < 2; ++u) {
         if (u >= p.n_kb1) break;
-#pragma unroll
-        for (int i = 0; i < 10; ++i) {
-          const int idx = lw * 10 + i;
-          const int row = (idx / 5) * 16 + r_lo;
-          const int ch = (idx % 5) * 2 + c_lo;
-          const float4 x = v[u][i];
-          float4 hi, lo;
-          hi.x = __uint_as_float(__float_as_uint(x.x) & 0xFFFFE000u);
-          hi.y = __uint_as_float(__float_as_uint(x.y) & 0xFFFFE000u);
-          hi.z = __uint_as_float(__float_as_uint(x.z) & 0xFFFFE000u);
-          hi.w = __uint_as_float(__float_as_uint(x.w) & 0xFFFFE000u);
-          lo.x = x.x - hi.x; lo.y = x.y - hi.y;
-          lo.z = x.z - hi.z; lo.w = x.w - hi.w;
-          const uint32_t off =
-              (uint32_t)(ch * (kTileM / 8) + (row >> 3)) * 128u + (row & 7) * 16u;
-          unsigned char* a = xa + (size_t)u * kABlock + off;
-          *reinterpret_cast<float4*>(a) = hi;
-          *reinterpret_cast<float4*>(a + kAPart) = lo;
-        }
+        store_kblock(xa + (size_t)u * kABlock, v[u], lw, lane);
       }
       fence_proxy_async();
       mbar_arrive(bar_xfull);
-      if (threadIdx.x == 128) FTRACE_L(0, 120 + ti);
+      if (threadIdx.x == 128) TRACE(0, 120 + ti);
     };
     for (int ti = 0; ti < n_my; ++ti) load_x(ti);
   } else if (warp == 13) {
@@ -245,7 +180,7 @@ __global__ void __launch_bounds__(kThreads, 1) ffn_tf32_kernel(const Params p) {
           bytes = w2_stage;
         }
         mbar_wait(bar_wempty + 8u * s, ph ^ 1u);
-        if (lane == 0) FTRACE_L(1, 1000 + it);
+        if (lane == 0) TRACE(1, 1000 + it);
         if (elect_one()) {
           mbar_arrive_expect_tx(bar_wfull + 8u * s, bytes);
           bulk_g2s(wr_base + s * wstage, src, bytes, bar_wfull + 8u * s);
@@ -257,91 +192,64 @@ __global__ void __launch_bounds__(kThreads, 1) ffn_tf32_kernel(const Params p) {
     // =============================== MMA issue ===============================
     // the whole warp walks the loop (all lanes poll the barriers); one elected
     // lane issues -- see elect_one() for why not `if (lane == 0)`
-    {
-      // kind::tf32, fp32 accumulate, A and B K-major, M = 128
-      const uint32_t idesc1 = (1u << 4) | (2u << 7) | (2u << 10) |
-                              ((uint32_t)(kHC >> 3) << 17) | (8u << 24);
-      const uint32_t idesc2 = (1u << 4) | (2u << 7) | (2u << 10) |
-                              ((uint32_t)(npad >> 3) << 17) | (8u << 24);
-      const uint32_t lbo_b1 = (uint32_t)kHC * 16u, lbo_b2 = (uint32_t)npad * 16u;
-      const uint32_t w1_part = (uint32_t)kHC * kKB * 4;
-      const uint32_t w2_part = (uint32_t)npad * kKB * 4;
-      const uint32_t d_y = tmem_base + (uint32_t)p.hidden;
-      const uint32_t d_lo = d_y + (uint32_t)npad;
-      uint32_t it = 0, hu = 0;   // weight stage counter, hidden K-block counter
-      for (int ti = 0; ti < n_my; ++ti) {
-        if (lane == 0) FTRACE_L(2, 200 + ti);
-        mbar_wait(bar_xfull, ti & 1);
-        tc_fence_after();
-        if (lane == 0) FTRACE_L(2, 210 + ti);
-        // ---- GEMM1: H chunk c = X . W1[80c : 80c + 80]^T ----
-        for (int c = 0; c < p.n_hc; ++c) {
-          const uint32_t d = tmem_base + (uint32_t)(c * kHC);
-          for (int kb = 0; kb < p.n_kb1; ++kb, ++it) {
-            const uint32_t s = it % S, ph = (it / S) & 1u;
-            mbar_wait(bar_wfull + 8u * s, ph);
-            tc_fence_after();
-            if (lane == 0) FTRACE_L(2, 2000 + it);
-            const uint32_t a_hi = xa_base + (uint32_t)kb * kABlock;
-            const uint32_t a_lo = a_hi + kAPart;
-            const uint32_t w_hi = wr_base + s * wstage;
-            const uint32_t w_lo = w_hi + w1_part;
-            if (elect_one()) {
-#pragma unroll
-            for (int k = 0; k < kChunks / 2; ++k) {
-              const uint32_t ao = 2u * k * kAChunkStride, bo = 2u * k * lbo_b1;
-              const uint64_t dah = smem_desc(a_hi + ao, kAChunkStride, 128);
-              const uint64_t dal = smem_desc(a_lo + ao, kAChunkStride, 128);
-              const uint64_t dbh = smem_desc(w_hi + bo, lbo_b1, 128);
-              const uint64_t dbl = smem_desc(w_lo + bo, lbo_b1, 128);
-              mma_tf32(d, dah, dbh, idesc1, (kb | k) != 0);
-              mma_tf32(d, dal, dbh, idesc1, 1u);
-              mma_tf32(d, dah, dbl, idesc1, 1u);
-            }
+    const uint32_t idesc1 = idesc_tf32_m128(kHC);
+    const uint32_t idesc2 = idesc_tf32_m128(npad);
+    const uint32_t lbo_b1 = (uint32_t)kHC * 16u, lbo_b2 = (uint32_t)npad * 16u;
+    const uint32_t w1_part = (uint32_t)kHC * kKB * 4;
+    const uint32_t w2_part = (uint32_t)npad * kKB * 4;
+    const uint32_t d_y = tmem_base + (uint32_t)p.hidden;
+    const uint32_t d_lo = d_y + (uint32_t)npad;
+    uint32_t it = 0, hu = 0;   // weight stage counter, hidden K-block counter
+    for (int ti = 0; ti < n_my; ++ti) {
+      if (lane == 0) TRACE(2, 200 + ti);
+      mbar_wait(bar_xfull, ti & 1);
+      tc_fence_after();
+      if (lane == 0) TRACE(2, 210 + ti);
+      // ---- GEMM1: H chunk c = X . W1[80c : 80c + 80]^T ----
+      for (int c = 0; c < p.n_hc; ++c) {
+        const uint32_t d = tmem_base + (uint32_t)(c * kHC);
+        for (int kb = 0; kb < p.n_kb1; ++kb, ++it) {
+          const uint32_t s = it % S, ph = (it / S) & 1u;
+          mbar_wait(bar_wfull + 8u * s, ph);
+          tc_fence_after();
+          if (lane == 0) TRACE(2, 2000 + it);
+          const uint32_t w_hi = wr_base + s * wstage;
+          if (elect_one()) {
+            mma_kblock_ss(d, xa_base + (uint32_t)kb * kABlock, w_hi, w_hi + w1_part,
+                          lbo_b1, idesc1, kb);
             tc_commit(bar_wempty + 8u * s);
             if (kb == p.n_kb1 - 1) {
               tc_commit(bar_hfull + 8u * c);    // chunk c can be converted
               if (c == p.n_hc - 1) tc_commit(bar_xempty);   // X tile consumed
             }
-            }
-            __syncwarp();
-          }
-        }
-        // ---- GEMM2: Y += Hblk . W2blk^T ----
-        mbar_wait(bar_yempty, (ti & 1) ^ 1);    // Y of the previous tile drained
-        tc_fence_after();
-        for (int kb = 0; kb < p.n_kb2; ++kb, ++it, ++hu) {
-          const uint32_t s = it % S, ph = (it / S) & 1u;
-          const uint32_t g = (uint32_t)kb & 1u, hph = (hu >> 1) & 1u;
-          mbar_wait(bar_wfull + 8u * s, ph);
-          if (lane == 0) FTRACE_L(2, 2000 + it);
-          mbar_wait(bar_hafull + 8u * g, hph);
-          tc_fence_after();
-          if (lane == 0) FTRACE_L(2, 3000 + it);
-          // A from tensor memory: hi where GEMM1 left the K-block (converted
-          // in place), lo in ring stage g
-          const uint32_t a_hi = tmem_base + (uint32_t)(kb * kKB);
-          const uint32_t a_lo = d_lo + g * (uint32_t)kKB;
-          const uint32_t w_hi = wr_base + s * wstage;
-          const uint32_t w_lo = w_hi + w2_part;
-          if (elect_one()) {
-#pragma unroll
-          for (int k = 0; k < kChunks / 2; ++k) {
-            const uint32_t bo = 2u * k * lbo_b2;
-            const uint64_t dbh = smem_desc(w_hi + bo, lbo_b2, 128);
-            const uint64_t dbl = smem_desc(w_lo + bo, lbo_b2, 128);
-            mma_tf32_ts(d_y, a_hi + 8u * k, dbh, idesc2, (kb | k) != 0);
-            mma_tf32_ts(d_y, a_lo + 8u * k, dbh, idesc2, 1u);
-            mma_tf32_ts(d_y, a_hi + 8u * k, dbl, idesc2, 1u);
-          }
-          tc_commit(bar_wempty + 8u * s);
-          tc_commit(bar_haempty + 8u * g);
-          if (kb == p.n_kb2 - 1) tc_commit(bar_yfull);
           }
           __syncwarp();
         }
-        if (lane == 0) FTRACE_L(2, 220 + ti);
       }
+      // ---- GEMM2: Y += Hblk . W2blk^T ----
+      mbar_wait(bar_yempty, (ti & 1) ^ 1);    // Y of the previous tile drained
+      tc_fence_after();
+      for (int kb = 0; kb < p.n_kb2; ++kb, ++it, ++hu) {
+        const uint32_t s = it % S, ph = (it / S) & 1u;
+        const uint32_t g = (uint32_t)kb & 1u, hph = (hu >> 1) & 1u;
+        mbar_wait(bar_wfull + 8u * s, ph);
+        if (lane == 0) TRACE(2, 2000 + it);
+        mbar_wait(bar_hafull + 8u * g, hph);
+        tc_fence_after();
+        if (lane == 0) TRACE(2, 3000 + it);
+        // A from tensor memory: hi where GEMM1 left the K-block (converted
+        // in place), lo in ring stage g
+        const uint32_t w_hi = wr_base + s * wstage;
+        if (elect_one()) {
+          mma_kblock_ts(d_y, tmem_base + (uint32_t)(kb * kKB), d_lo + g * (uint32_t)kKB,
+                        w_hi, w_hi + w2_part, lbo_b2, idesc2, kb);
+          tc_commit(bar_wempty + 8u * s);
+          tc_commit(bar_haempty + 8u * g);
+          if (kb == p.n_kb2 - 1) tc_commit(bar_yfull);
+        }
+        __syncwarp();
+      }
+      if (lane == 0) TRACE(2, 220 + ti);
     }
     __syncwarp();
   } else if (warp != 13) {
@@ -358,10 +266,10 @@ __global__ void __launch_bounds__(kThreads, 1) ffn_tf32_kernel(const Params p) {
         for (int kb = 0; kb < p.n_kb2; ++kb, ++use) {
           const uint32_t g = use & 1u;       // == kb & 1 (n_kb2 is even)
           mbar_wait(bar_hfull + 8u * (kb / (kHC / kKB)), ti & 1);
-          if (threadIdx.x == 256) FTRACE_L(3, 4000 + use);
+          if (threadIdx.x == 256) TRACE(3, 4000 + use);
           mbar_wait(bar_haempty + 8u * g, ((use >> 1) & 1u) ^ 1u);
           tc_fence_after();
-          if (threadIdx.x == 256) FTRACE_L(3, 5000 + use);
+          if (threadIdx.x == 256) TRACE(3, 5000 + use);
           const uint32_t taddr = lane_base + (uint32_t)(kb * kKB);
           float v[kKB], lo[kKB];
           tmem_ld16(taddr, v);
@@ -370,12 +278,7 @@ __global__ void __launch_bounds__(kThreads, 1) ffn_tf32_kernel(const Params p) {
           tmem_ld_wait();
           const float* bias = s_b1 + kb * kKB;
 #pragma unroll
-          for (int c = 0; c < kKB; ++c) {
-            const float t = fmaxf(v[c] + bias[c], 0.f);
-            const float hi = __uint_as_float(__float_as_uint(t) & 0xFFFFE000u);
-            v[c] = hi;
-            lo[c] = t - hi;
-          }
+          for (int c = 0; c < kKB; ++c) tf32_split(fmaxf(v[c] + bias[c], 0.f), v[c], lo[c]);
           tmem_st16(taddr, v);
           tmem_st16(taddr + 16u, v + 16);
           tmem_st8(taddr + 32u, v + 32);
@@ -386,7 +289,7 @@ __global__ void __launch_bounds__(kThreads, 1) ffn_tf32_kernel(const Params p) {
           tmem_st_wait();
           tc_fence_before();
           mbar_arrive(bar_hafull + 8u * g);
-          if (threadIdx.x == 256) FTRACE_L(3, 6000 + use);
+          if (threadIdx.x == 256) TRACE(3, 6000 + use);
         }
       }
     } else {
@@ -398,101 +301,31 @@ __global__ void __launch_bounds__(kThreads, 1) ffn_tf32_kernel(const Params p) {
       const int nc16 = npad >> 4;
       for (int ti = 0; ti < n_my; ++ti) {
         const int row0 = row_begin + ti * kTileM;
-        const bool in_range = row0 + gt < row_end;
         bulk_wait_read0();   // my row of the previous tile has left the slab
         asm volatile("bar.sync 1, 128;" ::: "memory");   // ... and everybody's
         // residual rows of this tile -> slab with cp.async while the tensor
         // pipe is still on the tile (4 lanes per row, 64 contiguous bytes per
         // row and round: coalesced; a load per thread and row inside the pass
         // below cost a full L2 round trip each: 6 us per tile)
-        if (p.residual) {
-          const int crow = gt >> 2, cq = gt & 3;
-#pragma unroll 1
-          for (int c = 0; c < nc16; ++c) {
-            const int col = 16 * c + 4 * cq;
-#pragma unroll
-            for (int i = 0; i < 4; ++i) {
-              const int r = crow + 32 * i;
-              const bool ok = row0 + r < row_end && col < E;
-              const float* src = p.residual +
-                                 (size_t)(ok ? row0 + r : row_begin) * p.ldr +
-                                 (ok ? col : 0);
-              const uint32_t dst = smem_u32(slab + (size_t)r * pitch + col);
-              asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;" ::"r"(dst),
-                           "l"(src), "r"(ok ? 16 : 0)
-                           : "memory");
-            }
-          }
-          asm volatile("cp.async.commit_group;" ::: "memory");
-        }
-        if (threadIdx.x == 0) FTRACE_L(4, 300 + ti);
+        if (p.residual)
+          prefetch_rows(slab, pitch, p.residual, p.ldr, row0, row_end, row_begin,
+                        E, nc16, gt);
+        if (threadIdx.x == 0) TRACE(4, 300 + ti);
         mbar_wait(bar_yfull, ti & 1);
         tc_fence_after();
-        if (threadIdx.x == 0) FTRACE_L(4, 310 + ti);
+        if (threadIdx.x == 0) TRACE(4, 310 + ti);
         if (p.residual) {
-          asm volatile("cp.async.wait_group 0;" ::: "memory");
+          cp_async_wait0();
           asm volatile("bar.sync 1, 128;" ::: "memory");
         }
-        float sum = 0.f, sq = 0.f, shiftK = 0.f;
-#pragma unroll 1
-        for (int c = 0; c < nc16; ++c) {
-          float v[16];
-          tmem_ld16(ty + 16u * c, v);
-          tmem_ld_wait();
-          if (c == nc16 - 1) {
-            tc_fence_before();
-            mbar_arrive(bar_yempty);
-          }
-#pragma unroll
-          for (int j = 0; j < 4; ++j) {
-            const int col = 16 * c + 4 * j;
-            if (col < E) {
-              const float4 bb = *reinterpret_cast<const float4*>(s_b2 + col);
-              float4 t = make_float4(v[4 * j] + bb.x, v[4 * j + 1] + bb.y,
-                                     v[4 * j + 2] + bb.z, v[4 * j + 3] + bb.w);
-              float4* cell = reinterpret_cast<float4*>(my_row + col);
-              if (p.residual) {
-                const float4 r = *cell;
-                t.x += r.x; t.y += r.y; t.z += r.z; t.w += r.w;
-              }
-              *cell = t;
-              if (col == 0) shiftK = t.x;
-              const float a = t.x - shiftK, b = t.y - shiftK, cc = t.z - shiftK,
-                          d = t.w - shiftK;
-              sum += (a + b) + (cc + d);
-              sq += (a * a + b * b) + (cc * cc + d * d);
-            }
-          }
-        }
-        if (p.gamma) {
-          const float dm = sum / (float)E;
-          const float mean = shiftK + dm;
-          const float var = fmaxf(sq / (float)E - dm * dm, 0.f);
-          const float rstd = rsqrtf(var + p.eps);
-          const float4* g4 = reinterpret_cast<const float4*>(s_gamma);
-          const float4* b4 = reinterpret_cast<const float4*>(s_beta);
-#pragma unroll 4
-          for (int j = 0; j < (E >> 2); ++j) {
-            float4* cell = reinterpret_cast<float4*>(my_row + 4 * j);
-            const float4 t = *cell, g = g4[j], b = b4[j];
-            *cell = make_float4(fmaf((t.x - mean) * rstd, g.x, b.x),
-                                fmaf((t.y - mean) * rstd, g.y, b.y),
-                                fmaf((t.z - mean) * rstd, g.z, b.z),
-                                fmaf((t.w - mean) * rstd, g.w, b.w));
-          }
-        }
-        // the finished row leaves as ONE bulk (TMA) store issued by its own
-        // thread (its own STS are ordered before the copy by the proxy fence)
-        if (in_range) {
-          fence_proxy_async();
-          bulk_s2g(p.y + (size_t)(row0 + gt) * p.ldy, smem_u32(my_row),
-                   (uint32_t)E * 4u);
-        }
-        bulk_commit();
-        if (threadIdx.x == 0) FTRACE_L(4, 320 + ti);
+        const RowStats st =
+            ln_pass1(ty, nc16, E, s_b2, false, p.residual, my_row, bar_yempty);
+        if (p.gamma) ln_normalise(my_row, E, st, p.eps, s_gamma, s_beta);
+        store_row(p.y, p.ldy, row0 + gt, row_end, my_row, E);
+        if (threadIdx.x == 0) TRACE(4, 320 + ti);
       }
       bulk_wait0();
-      if (threadIdx.x == 0) FTRACE_L(4, 330);
+      if (threadIdx.x == 0) TRACE(4, 330);
     }
   }
 
@@ -500,33 +333,25 @@ __global__ void __launch_bounds__(kThreads, 1) ffn_tf32_kernel(const Params p) {
   __syncthreads();
   if (warp == 12) {
     tc_fence_after();
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(
-                     tmem_base),
-                 "r"(kTmemCols)
-                 : "memory");
+    tmem_dealloc(tmem_base);
   }
 }
-
-static inline int pad16(int n) { return (n + 15) / 16 * 16; }
 
 }  // namespace ffn
 }  // namespace fbbev
 
 using namespace fbbev;
 
-#ifdef FFN_TRACE
-FBBEV_API int fbbev_debug_ffn_trace(long long* out, int* counts) {
-  cudaMemcpyFromSymbol(counts, ffn::g_ffn_trace_cnt, sizeof(int) * 5);
-  cudaMemcpyFromSymbol(out, ffn::g_ffn_trace,
-                       sizeof(long long) * 5 * 2 * ffn::kTraceCap);
-  return ffn::kTraceCap;
+#ifdef TC_TRACE
+int fbbev::ffn_trace_copy(long long* out, int* counts) {
+  return tc_trace_copy(out, counts);
 }
 #endif
 
 FBBEV_API int fbbev_ffn_supported(int32_t embed, int32_t hidden) {
   return embed > 0 && embed <= ffn::kMaxE && embed % 4 == 0 && hidden > 0 &&
                  hidden % ffn::kHC == 0 &&
-                 hidden + ffn::pad16(embed) + 2 * ffn::kKB <= ffn::kTmemCols &&
+                 hidden + pad16(embed) + 2 * kKB <= kTmemCols &&
                  hidden <= ffn::kMaxHidden
              ? 1
              : 0;
@@ -557,43 +382,30 @@ FBBEV_API int fbbev_ffn_fwd(const float* x, int64_t ldx, const float* w1_packed,
   ffn::Params p;
   p.x = x; p.w1p = w1_packed; p.b1 = b1; p.w2p = w2_packed; p.b2 = b2;
   p.residual = residual; p.gamma = ln_weight; p.beta = ln_bias; p.y = y;
-  p.M = (int)m; p.E = embed; p.hidden = hidden; p.npad = ffn::pad16(embed);
-  p.n_kb1 = (embed + ffn::kKB - 1) / ffn::kKB;
-  p.n_kb2 = hidden / ffn::kKB;
+  p.M = (int)m; p.E = embed; p.hidden = hidden; p.npad = pad16(embed);
+  p.n_kb1 = (embed + kKB - 1) / kKB;
+  p.n_kb2 = hidden / kKB;
   p.n_hc = hidden / ffn::kHC;
   p.ldx = ldx; p.ldr = ldr; p.ldy = ldy; p.eps = ln_eps;
-  const size_t w1_stage = 2 * (size_t)ffn::kHC * ffn::kKB * 4;
-  const size_t w2_stage = 2 * (size_t)p.npad * ffn::kKB * 4;
+  const size_t w1_stage = 2 * (size_t)ffn::kHC * kKB * 4;
+  const size_t w2_stage = 2 * (size_t)p.npad * kKB * 4;
   const size_t wstage = w1_stage > w2_stage ? w1_stage : w2_stage;
   const size_t fixed =
       2 * (size_t)ffn::kABlock + ffn::kSlabBytes + ffn::kCtrlBytes;
-  int S = (int)((ffn::kSmemLimit - fixed) / wstage);
+  int S = (int)((kSmemLimit - fixed) / wstage);
   S = S > 4 ? 4 : S;
   if (S < 2) return FBBEV_ERR_UNSUPPORTED;
   p.wstages = S;
   const size_t smem = fixed + (size_t)S * wstage;
-  static int n_sm = 0;
-  if (n_sm == 0) {
-    int dev = 0;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, dev);
-    if (n_sm <= 0) n_sm = 148;
-  }
+  const int n_sm = sm_count();
   // whole tiles per CTA: every tile costs one pass over the weights (410 KB
   // from L2) whatever its row count, so 105 CTAs x 3 full tiles beat 148 CTAs
   // x (2 full + 1 sliver) for 40000 rows: same makespan, 30 % less L2 traffic
-  const int n_tiles = (int)ceil_div64(m, ffn::kTileM);
+  const int n_tiles = (int)ceil_div64(m, kTileM);
   const int tiles_per_cta = (int)ceil_div64(n_tiles, n_sm);
-  p.rows_per_cta = tiles_per_cta * ffn::kTileM;
+  p.rows_per_cta = tiles_per_cta * kTileM;
   const int grid = (int)ceil_div64(m, p.rows_per_cta);
-  static size_t allowed = 0;
-  if (smem > allowed) {
-    cudaError_t e = cudaFuncSetAttribute(
-        ffn::ffn_tf32_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-        (int)smem);
-    if (e != cudaSuccess) return (int)e;
-    allowed = smem;
-  }
+  if (const int e = raise_smem_limit<ffn::ffn_tf32_kernel>(smem)) return e;
   count_launch();
   ffn::ffn_tf32_kernel<<<grid, ffn::kThreads, smem, as_stream(stream)>>>(p);
   return launch_status();

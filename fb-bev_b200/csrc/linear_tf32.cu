@@ -34,44 +34,18 @@
 //               dependent issue), hence two groups.
 //   Ring of K-blocks of 40 floats (5 k-steps) between loaders and MMA, two
 //   accumulators in TMEM between MMA and epilogue.
-#include "common.cuh"
 #include "tc5.cuh"
 
 namespace fbbev {
 
-constexpr int kKB = 40;                          // floats of K per stage
-constexpr int kChunks = kKB / 4;                 // 16-byte chunks per row
-constexpr int kTileM = 128;
-constexpr int kAPart = kTileM * kKB * 4;         // bytes of A_hi (== A_lo)
-constexpr int kAChunkStride = (kTileM / 8) * 128;  // bytes between K chunks
 constexpr int kLinThreads = 448;  // 14 warps, see the role table above
 constexpr int kMaxN = 192;
-constexpr int kTmemCols = 512;
-constexpr int kSmemLimit = 232448 - 1024;
 constexpr int kSlabPitch = 20;  // floats: 16 columns + 4 (bank spread)
 constexpr int kSlabBytes = 2 * kTileM * kSlabPitch * 4;  // both groups
 // control area after the stages: mbarriers + TMEM slot (256 B), then bias /
 // LayerNorm weight / LayerNorm bias staged once (the L1 left beside ~220 KB of
 // shared memory is too small to keep them: a __ldg would be an L2 round trip)
 constexpr int kCtrlBytes = 256 + 3 * kMaxN * 4;
-
-#ifdef LIN_TRACE
-// timeline of CTA 0: every tracing thread appends (tag, clock) to its own
-// shared-memory lane; dumped to global memory at the end of the kernel
-__device__ long long g_trace[512];
-__device__ int g_trace_n;
-#define TRACE_DECL __shared__ long long s_trace[8][64]; __shared__ int s_trace_n[8];
-#define TRACE(lane_, tag)                                                    \
-  do {                                                                       \
-    if (blockIdx.x == 0) {                                                   \
-      const int ti_ = s_trace_n[lane_]++;                                    \
-      if (ti_ < 32) { s_trace[lane_][2 * ti_] = (tag); s_trace[lane_][2 * ti_ + 1] = clock64(); } \
-    }                                                                        \
-  } while (0)
-#else
-#define TRACE_DECL
-#define TRACE(lane_, tag) do {} while (0)
-#endif
 
 // ------------------------------ weight packing -------------------------------
 // W [N][K] row-major -> [k-block][hi, lo][chunk 0..9][Npad / 8][8 rows][4]:
@@ -89,13 +63,10 @@ __global__ void linear_pack_kernel(const float* __restrict__ w, int n, int k,
 #pragma unroll
     for (int j = 0; j < 4; ++j) {
       const int col = kb * kKB + ch * 4 + j;
-      const float v = (row < n && col < k) ? w[(int64_t)row * k + col] : 0.f;
-      hi[j] = __uint_as_float(__float_as_uint(v) & 0xFFFFE000u);
-      lo[j] = v - hi[j];
+      tf32_split((row < n && col < k) ? w[(int64_t)row * k + col] : 0.f, hi[j], lo[j]);
     }
     const int64_t part = (int64_t)kChunks * npad * 4;  // floats of one hi / lo part
-    const int64_t off =
-        (int64_t)kb * 2 * part + (int64_t)ch * npad * 4 + (row / 8) * 32 + (row % 8) * 4;
+    const int64_t off = (int64_t)kb * 2 * part + kmajor_off(row, ch, npad) / 4;
     *reinterpret_cast<float4*>(out + off) = make_float4(hi[0], hi[1], hi[2], hi[3]);
     *reinterpret_cast<float4*>(out + off + part) =
         make_float4(lo[0], lo[1], lo[2], lo[3]);
@@ -128,9 +99,6 @@ __global__ void __launch_bounds__(kLinThreads, 1)
     linear_tf32_kernel(const LinearParams p) {
   extern __shared__ __align__(1024) unsigned char smem[];
   TRACE_DECL
-#ifdef LIN_TRACE
-  if (threadIdx.x < 8) s_trace_n[threadIdx.x] = 0;
-#endif
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int npad = p.npad, S = p.stages;
   const uint32_t w_part = (uint32_t)npad * kKB * 4;        // bytes of W_hi
@@ -157,13 +125,7 @@ __global__ void __launch_bounds__(kLinThreads, 1)
       fence_mbar_init();
     }
     __syncwarp();
-    asm volatile(
-        "tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(
-            smem_u32(tmem_slot)),
-        "r"(kTmemCols)
-        : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::
-                     : "memory");
+    tmem_alloc(smem_u32(tmem_slot));
   }
   float* s_bias = reinterpret_cast<float*>(ctrl + 256);
   float* s_gamma = s_bias + kMaxN;
@@ -177,7 +139,7 @@ __global__ void __launch_bounds__(kLinThreads, 1)
   __syncthreads();
   tc_fence_after();
   const uint32_t tmem_base = *tmem_slot;
-  if (threadIdx.x == 0) TRACE(0, 1);
+  if (threadIdx.x == 0) TRACE(3, 1);
   // this CTA's rows and 128-row tiles (the last one may be partial)
   const int row_begin = blockIdx.x * p.rows_per_cta;
   const int row_end = min(p.M, row_begin + p.rows_per_cta);
@@ -186,7 +148,6 @@ __global__ void __launch_bounds__(kLinThreads, 1)
   if (warp >= 4 && warp < 8) {
     // ================================ loaders ================================
     const int lw = warp - 4;
-    const int r_lo = lane & 15, c_lo = lane >> 4;
     const int total = n_my * p.n_kb;  // (tile, K-block) items, two per round
     for (int w0 = 0; w0 < total; w0 += 2) {
       float4 v[2][10];
@@ -194,38 +155,8 @@ __global__ void __launch_bounds__(kLinThreads, 1)
       for (int u = 0; u < 2; ++u) {
         const int w = w0 + u;
         const int ti = w / p.n_kb, kb = w - ti * p.n_kb;
-        // rows (2 lw + h) * 16 + r_lo, h = 0 / 1; columns kb*40 + 8 cp + 4 c_lo
-        const int g0 = row_begin + ti * kTileM + lw * 32 + r_lo;
-        const int col0 = kb * kKB + 4 * c_lo;
-        const float* b0 = p.x + (size_t)g0 * p.ldx + col0;
-        const float* b1 = b0 + (size_t)16 * p.ldx;
-        const bool ok0 = w < total && g0 < row_end;
-        const bool ok1 = w < total && g0 + 16 < row_end;
-#pragma unroll
-        for (int i = 0; i < 10; ++i) {
-          const int cp = i % 5;
-          const bool ok = (i < 5 ? ok0 : ok1) && col0 + 8 * cp < p.K;
-          v[u][i] = ok ? __ldg(reinterpret_cast<const float4*>(
-                             (i < 5 ? b0 : b1) + 8 * cp))
-                       : make_float4(0.f, 0.f, 0.f, 0.f);
-        }
-        if (p.x_add) {  // query + query_pos in the loader (one fp32 add, as torch)
-          const float* a0 = p.x_add + (size_t)g0 * p.ldxa + col0;
-          const float* a1 = a0 + (size_t)16 * p.ldxa;
-#pragma unroll
-          for (int i = 0; i < 10; ++i) {
-            const int cp = i % 5;
-            const bool ok = (i < 5 ? ok0 : ok1) && col0 + 8 * cp < p.K;
-            if (ok) {
-              const float4 a = __ldg(reinterpret_cast<const float4*>(
-                  (i < 5 ? a0 : a1) + 8 * cp));
-              v[u][i].x = __fadd_rn(v[u][i].x, a.x);
-              v[u][i].y = __fadd_rn(v[u][i].y, a.y);
-              v[u][i].z = __fadd_rn(v[u][i].z, a.z);
-              v[u][i].w = __fadd_rn(v[u][i].w, a.w);
-            }
-          }
-        }
+        gather_kblock(v[u], p.x, p.ldx, p.x_add, p.ldxa, p.K,
+                      row_begin + ti * kTileM, row_end, kb, w < total, lw, lane);
       }
       if (threadIdx.x == 128) TRACE(1, 100 + w0);
       for (int u = 0; u < 2; ++u) {
@@ -234,25 +165,7 @@ __global__ void __launch_bounds__(kLinThreads, 1)
         const uint32_t s = it % S, ph = (it / S) & 1u;
         mbar_wait(bar_empty + 8u * s, ph ^ 1u);
         if (threadIdx.x == 128) TRACE(1, 200 + it);
-#pragma unroll
-        for (int i = 0; i < 10; ++i) {
-          const int idx = lw * 10 + i;
-          const int row = (idx / 5) * 16 + r_lo;
-          const int ch = (idx % 5) * 2 + c_lo;
-          const float4 x = v[u][i];
-          float4 hi, lo;
-          hi.x = __uint_as_float(__float_as_uint(x.x) & 0xFFFFE000u);
-          hi.y = __uint_as_float(__float_as_uint(x.y) & 0xFFFFE000u);
-          hi.z = __uint_as_float(__float_as_uint(x.z) & 0xFFFFE000u);
-          hi.w = __uint_as_float(__float_as_uint(x.w) & 0xFFFFE000u);
-          lo.x = x.x - hi.x; lo.y = x.y - hi.y;
-          lo.z = x.z - hi.z; lo.w = x.w - hi.w;
-          const uint32_t off =
-              (uint32_t)(ch * (kTileM / 8) + (row >> 3)) * 128u + (row & 7) * 16u;
-          unsigned char* a = smem + (size_t)s * stage_bytes + off;
-          *reinterpret_cast<float4*>(a) = hi;
-          *reinterpret_cast<float4*>(a + kAPart) = lo;
-        }
+        store_kblock(smem + (size_t)s * stage_bytes, v[u], lw, lane);
         fence_proxy_async();
         mbar_arrive(bar_full + 8u * s);
         if (threadIdx.x == 128) TRACE(1, 300 + it);
@@ -278,45 +191,29 @@ __global__ void __launch_bounds__(kLinThreads, 1)
     // elected lane issues: under a divergent `if (lane == 0)` the compiler
     // wraps every UTCHMMA in an ELECT / BRA.U.ANY serialisation loop (see
     // elect_one(), tc5.cuh) -- ~100 instead of ~52 cycles per MMA.
-    {
-      // kind::tf32, fp32 accumulate, A and B K-major, M = 128, N = npad
-      const uint32_t idesc = (1u << 4) | (2u << 7) | (2u << 10) |
-                             ((uint32_t)(npad >> 3) << 17) | (8u << 24);
-      const uint32_t lbo_b = (uint32_t)npad * 16u;
-      uint32_t it = 0, tc = 0;
-      for (int ti = 0; ti < n_my; ++ti, ++tc) {
-        const uint32_t acc = tc & 1u, aph = (tc >> 1) & 1u;
-        mbar_wait(bar_tempty + 8u * acc, aph ^ 1u);
+    const uint32_t idesc = idesc_tf32_m128(npad);
+    const uint32_t lbo_b = (uint32_t)npad * 16u;
+    uint32_t it = 0, tc = 0;
+    for (int ti = 0; ti < n_my; ++ti, ++tc) {
+      const uint32_t acc = tc & 1u, aph = (tc >> 1) & 1u;
+      mbar_wait(bar_tempty + 8u * acc, aph ^ 1u);
+      tc_fence_after();
+      const uint32_t d = tmem_base + acc * (uint32_t)npad;
+      for (int kb = 0; kb < p.n_kb; ++kb, ++it) {
+        const uint32_t s = it % S, ph = (it / S) & 1u;
+        mbar_wait(bar_full + 8u * s, ph);
         tc_fence_after();
-        const uint32_t d = tmem_base + acc * (uint32_t)npad;
-        for (int kb = 0; kb < p.n_kb; ++kb, ++it) {
-          const uint32_t s = it % S, ph = (it / S) & 1u;
-          mbar_wait(bar_full + 8u * s, ph);
-          tc_fence_after();
-          if (lane == 0) TRACE(2, 400 + it);
-          const uint32_t a_hi = smem_base + s * stage_bytes;
-          const uint32_t a_lo = a_hi + kAPart;
-          const uint32_t w_hi = a_lo + kAPart;
-          const uint32_t w_lo = w_hi + w_part;
-          if (elect_one()) {
-#pragma unroll
-            for (int k = 0; k < kChunks / 2; ++k) {
-              const uint32_t ao = 2u * k * kAChunkStride, bo = 2u * k * lbo_b;
-              const uint64_t dah = smem_desc(a_hi + ao, kAChunkStride, 128);
-              const uint64_t dal = smem_desc(a_lo + ao, kAChunkStride, 128);
-              const uint64_t dbh = smem_desc(w_hi + bo, lbo_b, 128);
-              const uint64_t dbl = smem_desc(w_lo + bo, lbo_b, 128);
-              mma_tf32(d, dah, dbh, idesc, (kb | k) != 0);
-              mma_tf32(d, dal, dbh, idesc, 1u);
-              mma_tf32(d, dah, dbl, idesc, 1u);
-            }
-            tc_commit(bar_empty + 8u * s);
-            if (kb == p.n_kb - 1) tc_commit(bar_tfull + 8u * acc);
-          }
-          __syncwarp();
+        if (lane == 0) TRACE(2, 400 + it);
+        const uint32_t a_hi = smem_base + s * stage_bytes;
+        const uint32_t w_hi = a_hi + 2u * kAPart;
+        if (elect_one()) {
+          mma_kblock_ss(d, a_hi, w_hi, w_hi + w_part, lbo_b, idesc, kb);
+          tc_commit(bar_empty + 8u * s);
+          if (kb == p.n_kb - 1) tc_commit(bar_tfull + 8u * acc);
         }
-        if (lane == 0) TRACE(2, 500 + tc);
+        __syncwarp();
       }
+      if (lane == 0) TRACE(2, 500 + tc);
     }
     __syncwarp();
   } else {
@@ -356,100 +253,23 @@ __global__ void __launch_bounds__(kLinThreads, 1)
       if (LN) {
         bulk_wait_read0();  // this thread's row of the previous tile has left
         group_sync();       // ... and so have all the others
-        if (p.residual) {
-#pragma unroll 1
-          for (int c = 0; c < nc16; ++c) {
-            const int col = 16 * c + 4 * cq;
-#pragma unroll
-            for (int i = 0; i < 4; ++i) {
-              const int r = crow + 32 * i;
-              const bool ok = row0 + r < row_end && col < N;
-              const float* src = p.residual +
-                                 (size_t)(ok ? row0 + r : row_begin) * p.ldr +
-                                 (ok ? col : 0);
-              const uint32_t dst = smem_u32(slab + (size_t)r * pitch + col);
-              asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;" ::"r"(dst),
-                           "l"(src), "r"(ok ? 16 : 0)
-                           : "memory");
-            }
-          }
-          asm volatile("cp.async.commit_group;" ::: "memory");
-        }
+        if (p.residual)
+          prefetch_rows(slab, pitch, p.residual, p.ldr, row0, row_end, row_begin,
+                        N, nc16, gt);
         if (gt == 0) TRACE(3 + grp, 600 + tc);
         mbar_wait(bar_tfull + 8u * grp, aph);
         tc_fence_after();
         if (gt == 0) TRACE(3 + grp, 700 + tc);
         if (p.residual) {
-          asm volatile("cp.async.wait_group 0;" ::: "memory");
+          cp_async_wait0();
           group_sync();
         }
-        // pass 1: accumulator + bias (+ ReLU) + residual -> my slab row; sum and
-        // sum of squares about a shift K = the row's first element (a one-pass
-        // variance that does not cancel: |mean - K| is a few sigma at most)
-        float sum = 0.f, sq = 0.f, shiftK = 0.f;
-#pragma unroll 1
-        for (int c = 0; c < nc16; ++c) {
-          float v[16];
-          tmem_ld16(taddr + 16u * c, v);
-          tmem_ld_wait();
-          if (c == nc16 - 1) {
-            tc_fence_before();
-            mbar_arrive(bar_tempty + 8u * grp);
-          }
-#pragma unroll
-          for (int j = 0; j < 4; ++j) {
-            const int col = 16 * c + 4 * j;
-            if (col < N) {
-              const float4 bb = bias4[col >> 2];
-              float4 t = make_float4(v[4 * j] + bb.x, v[4 * j + 1] + bb.y,
-                                     v[4 * j + 2] + bb.z, v[4 * j + 3] + bb.w);
-              if (p.relu) {
-                t.x = fmaxf(t.x, 0.f); t.y = fmaxf(t.y, 0.f);
-                t.z = fmaxf(t.z, 0.f); t.w = fmaxf(t.w, 0.f);
-              }
-              float4* cell = reinterpret_cast<float4*>(my_row + col);
-              if (p.residual) {
-                const float4 r = *cell;
-                t.x += r.x; t.y += r.y; t.z += r.z; t.w += r.w;
-              }
-              *cell = t;
-              if (col == 0) shiftK = t.x;
-              const float a = t.x - shiftK, b = t.y - shiftK, cc = t.z - shiftK,
-                          d = t.w - shiftK;
-              sum += (a + b) + (cc + d);
-              sq += (a * a + b * b) + (cc * cc + d * d);
-            }
-          }
-        }
+        const RowStats st = ln_pass1(taddr, nc16, N, s_bias, p.relu, p.residual,
+                                     my_row, bar_tempty + 8u * grp);
         if (gt == 0) TRACE(3 + grp, 800 + tc);
-        // pass 2: normalise in place
-        const int c4 = N >> 2;
-        const float dm = sum / (float)N;       // mean - K
-        const float mean = shiftK + dm;
-        const float var = fmaxf(sq / (float)N - dm * dm, 0.f);
-        const float rstd = rsqrtf(var + p.eps);
-        const float4* g4 = reinterpret_cast<const float4*>(s_gamma);
-        const float4* b4 = reinterpret_cast<const float4*>(s_beta);
-#pragma unroll 4
-        for (int j = 0; j < c4; ++j) {
-          float4* cell = reinterpret_cast<float4*>(my_row + 4 * j);
-          const float4 t = *cell, g = g4[j], b = b4[j];
-          *cell = make_float4(fmaf((t.x - mean) * rstd, g.x, b.x),
-                              fmaf((t.y - mean) * rstd, g.y, b.y),
-                              fmaf((t.z - mean) * rstd, g.z, b.z),
-                              fmaf((t.w - mean) * rstd, g.w, b.w));
-        }
+        ln_normalise(my_row, N, st, p.eps, s_gamma, s_beta);
         if (gt == 0) TRACE(3 + grp, 900 + tc);
-        // the finished row leaves as ONE bulk (TMA) store issued by its own
-        // thread: N * 4 contiguous bytes in the slab and in y.  No barrier and
-        // no LDS / STG loop: the thread's own STS are ordered before its bulk
-        // copy by the proxy fence.
-        if (row0 + gt < row_end) {
-          fence_proxy_async();
-          bulk_s2g(p.y + (size_t)(row0 + gt) * p.ldy, smem_u32(my_row),
-                   (uint32_t)N * 4u);
-        }
-        bulk_commit();
+        store_row(p.y, p.ldy, row0 + gt, row_end, my_row, N);
         if (gt == 0) TRACE(3 + grp, 1000 + tc);
       } else {
         mbar_wait(bar_tfull + 8u * grp, aph);
@@ -515,43 +335,20 @@ __global__ void __launch_bounds__(kLinThreads, 1)
   if (LN) bulk_wait0();  // every row's bulk store has completed
   tc_fence_before();
   __syncthreads();
-  if (threadIdx.x == 0) TRACE(0, 2);
-#ifdef LIN_TRACE
-  __syncthreads();
-  if (blockIdx.x == 0 && threadIdx.x == 0) {
-    int n = 0;
-    for (int l = 0; l < 8; ++l)
-      for (int i = 0; i < min(s_trace_n[l], 32); ++i) {
-        g_trace[2 * n] = s_trace[l][2 * i];
-        g_trace[2 * n + 1] = s_trace[l][2 * i + 1];
-        ++n;
-      }
-    g_trace_n = n;
-  }
-#endif
+  if (threadIdx.x == 0) TRACE(3, 2);
   if (warp == 12) {
     tc_fence_after();
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(
-                     tmem_base),
-                 "r"(kTmemCols)
-                 : "memory");
+    tmem_dealloc(tmem_base);
   }
 }
 
-static inline int pad16(int n) { return (n + 15) / 16 * 16; }
 static inline int n_kblocks(int k) { return (k + kKB - 1) / kKB; }
 
-static int launch_linear(const LinearParams& p, bool ln, size_t smem, int grid,
+template <bool LN>
+static int launch_linear(const LinearParams& p, size_t smem, int grid,
                          cudaStream_t st) {
-  auto kern = ln ? linear_tf32_kernel<true> : linear_tf32_kernel<false>;
-  static size_t allowed[2] = {0, 0};
-  if (smem > allowed[ln]) {
-    cudaError_t e = cudaFuncSetAttribute(
-        kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    if (e != cudaSuccess) return (int)e;
-    allowed[ln] = smem;
-  }
-  kern<<<grid, kLinThreads, smem, st>>>(p);
+  if (const int e = raise_smem_limit<linear_tf32_kernel<LN>>(smem)) return e;
+  linear_tf32_kernel<LN><<<grid, kLinThreads, smem, st>>>(p);
   return launch_status();
 }
 
@@ -559,13 +356,10 @@ static int launch_linear(const LinearParams& p, bool ln, size_t smem, int grid,
 
 using namespace fbbev;
 
-#ifdef LIN_TRACE
-FBBEV_API int fbbev_debug_linear_trace(long long* out, int reset) {
-  int n = 0;
-  cudaMemcpyFromSymbol(&n, g_trace_n, sizeof(int));
-  cudaMemcpyFromSymbol(out, g_trace, sizeof(long long) * 512);
-  if (reset) { int z = 0; cudaMemcpyToSymbol(g_trace_n, &z, sizeof(int)); }
-  return n;
+#ifdef TC_TRACE
+// kernel 0: linear_tf32_kernel, 1: ffn_tf32_kernel (tools/tc_trace.py)
+FBBEV_API int fbbev_debug_tc_trace(int kernel, long long* out, int* counts) {
+  return kernel == 0 ? tc_trace_copy(out, counts) : ffn_trace_copy(out, counts);
 }
 #endif
 
@@ -637,13 +431,7 @@ static int linear_run(const float* x, int64_t ldx, const float* x_add,
   if (stages < 2) return FBBEV_ERR_UNSUPPORTED;
   p.stages = stages;
   const size_t smem = stages * stage + kCtrlBytes + slab_bytes;
-  static int n_sm = 0;
-  if (n_sm == 0) {
-    int dev = 0;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, dev);
-    if (n_sm <= 0) n_sm = 148;
-  }
+  const int n_sm = sm_count();
   // equal contiguous row ranges (multiples of 8 rows), one CTA per SM
   const int n_tiles = (int)ceil_div64(m, kTileM);
   int grid = n_tiles < n_sm ? n_tiles : n_sm;
@@ -651,7 +439,8 @@ static int linear_run(const float* x, int64_t ldx, const float* x_add,
   grid = (int)ceil_div64(m, p.rows_per_cta);
   cudaStream_t st = as_stream(stream);
   count_launch();
-  return launch_linear(p, ln, smem, grid, st);
+  return ln ? launch_linear<true>(p, smem, grid, st)
+            : launch_linear<false>(p, smem, grid, st);
 }
 
 FBBEV_API int fbbev_linear_fwd(const float* x, int64_t ldx, const float* packed,

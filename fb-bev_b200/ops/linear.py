@@ -14,19 +14,26 @@ from .. import _lib
 MAX_N = 192  # widest column block of one launch
 
 
-def _pack(weight):
-    """hi / lo split image of `weight` (n, k), one block per <= MAX_N columns.
-
-    Cached ON the weight tensor (so it dies with it and can never be mistaken
-    for another tensor's) and keyed by storage address and version counter, so
-    an optimizer step or ``load_state_dict`` triggers a re-pack."""
+def _cached(weight, attr, pack):
+    """``pack(weight as contiguous fp32)``, cached ON the weight tensor under
+    ``attr`` (so it dies with it and can never be mistaken for another
+    tensor's) and keyed by storage address and version counter, so an
+    optimizer step or ``load_state_dict`` triggers a re-pack."""
     key = (weight.data_ptr(), weight._version, tuple(weight.shape), weight.device)
-    hit = getattr(weight, "_fbbev_packed", None)
+    hit = getattr(weight, attr, None)
     if hit is not None and hit[0] == key:
         return hit[1]
+    packed = pack(weight.detach().contiguous().float())
+    try:
+        setattr(weight, attr, (key, packed))
+    except AttributeError:  # a tensor type without a __dict__: no caching
+        pass
+    return packed
+
+
+def _pack_blocks(w):
     L = _lib.lib()
-    n, k = weight.shape
-    w = weight.detach().contiguous().float()
+    n, k = w.shape
     blocks = []
     for n0 in range(0, n, MAX_N):
         n1 = min(n, n0 + MAX_N)
@@ -35,11 +42,12 @@ def _pack(weight):
         _lib.check(L.fbbev_linear_pack(_lib.ptr(w[n0:n1]), n1 - n0, k, _lib.ptr(buf),
                                        _lib.stream_ptr(w.device)), "fbbev_linear_pack")
         blocks.append((n0, n1, buf))
-    try:
-        weight._fbbev_packed = (key, blocks)
-    except AttributeError:  # a tensor type without a __dict__: no caching
-        pass
     return blocks
+
+
+def _pack(weight):
+    """hi / lo split image of `weight` (n, k), one block per <= MAX_N columns."""
+    return _cached(weight, "_fbbev_packed", _pack_blocks)
 
 
 def invalidate(obj):
@@ -167,28 +175,23 @@ def linear_pair(x, weight_a, bias_a, weight_b, bias_b, cache, x_add=None):
     return ya.view(*lead, na), yb.view(*lead, nb)
 
 
-def _pack_ffn_w1(weight):
-    """W1 (hidden, embed) as hidden / 80 separately packed 80-row blocks, one
-    buffer (the layout ``fbbev_ffn_fwd`` streams); cached like :func:`_pack`."""
-    key = (weight.data_ptr(), weight._version, tuple(weight.shape), weight.device)
-    hit = getattr(weight, "_fbbev_packed_ffn", None)
-    if hit is not None and hit[0] == key:
-        return hit[1]
+def _pack_w1_chunks(w):
     L = _lib.lib()
-    hidden, k = weight.shape
+    hidden, k = w.shape
     assert hidden % 80 == 0
-    w = weight.detach().contiguous().float()
     per = L.fbbev_linear_packed_bytes(80, k) // 4
     buf = torch.empty(per * (hidden // 80), dtype=torch.float32, device=w.device)
     for c in range(hidden // 80):
         _lib.check(L.fbbev_linear_pack(
             _lib.ptr(w[80 * c:80 * c + 80]), 80, k, _lib.ptr(buf[per * c:]),
             _lib.stream_ptr(w.device)), "fbbev_linear_pack")
-    try:
-        weight._fbbev_packed_ffn = (key, buf)
-    except AttributeError:
-        pass
     return buf
+
+
+def _pack_ffn_w1(weight):
+    """W1 (hidden, embed) as hidden / 80 separately packed 80-row blocks, one
+    buffer (the layout ``fbbev_ffn_fwd`` streams)."""
+    return _cached(weight, "_fbbev_packed_ffn", _pack_w1_chunks)
 
 
 def ffn_supported(x, w1, w2):

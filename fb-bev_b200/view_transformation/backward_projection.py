@@ -131,10 +131,8 @@ def _linear(mod, x, relu=False, residual=None, norm=None):
 def _linear_pair(owner, mod_a, mod_b, x, x_add=None):
     """``(mod_a(x + x_add), mod_b(x + x_add))`` for two nn.Linears on the same
     input, one launch when their widths allow (the addition happens in the
-    kernel's loader); set ``FBBEV_LINEAR_PAIR=0`` for two launches."""
-    if (os.environ.get('FBBEV_LINEAR_PAIR', '1') == '1'
-            and mod_a.weight.shape[1] % 4 == 0
-            and not torch.is_grad_enabled()):
+    kernel's loader)."""
+    if mod_a.weight.shape[1] % 4 == 0 and not torch.is_grad_enabled():
         return _linear_ops.linear_pair(
             x, mod_a.weight, mod_a.bias, mod_b.weight, mod_b.bias,
             owner.__dict__.setdefault('_pair_cache', {}), x_add=x_add)
@@ -253,7 +251,6 @@ class FFN(BaseModule):
                 if self.add_identity else None
             fc1, fc2 = self.layers[0][0], self.layers[-2]
             if (self.num_fcs == 2 and
-                    os.environ.get('FBBEV_FFN_FUSED', '1') == '1' and
                     _linear_ops.ffn_supported(x, fc1.weight, fc2.weight) and
                     (post_norm is None or
                      _linear_ops.ln_supported(fc2.weight.shape[0]))):

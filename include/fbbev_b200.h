@@ -550,7 +550,7 @@ int fbbev_linear_fwd_split(const float* x, int64_t ldx, const float* x_add,
  * w2_packed: fbbev_linear_pack(W2 (embed, hidden)).
  * b1 (hidden), b2 (embed), residual (m, embed; row stride ldr), ln_weight /
  * ln_bias (embed) may be NULL.  embed <= 80, embed % 4 == 0, hidden % 80 == 0,
- * hidden <= 400 (fbbev_ffn_supported); FBBEV_ERR_UNSUPPORTED otherwise (use
+ * hidden <= 320 (fbbev_ffn_supported); FBBEV_ERR_UNSUPPORTED otherwise (use
  * fbbev_linear_fwd per Linear).  Numerics as fbbev_linear_fwd (3xTF32).
  */
 int fbbev_ffn_supported(int32_t embed, int32_t hidden);
